@@ -21,7 +21,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree untouched (it may be read-only)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "distillation steps/sec (SD1.5 PCM-LoRA, bs=8/GPU)"
@@ -104,6 +106,32 @@ def synth_batch(cfg, B, hw, seed, pinned=True):
     if pinned and torch.cuda.is_available():
         t = {k: v.pin_memory() for k, v in t.items()}
     return t
+
+
+DUMP_SAMPLE = 1 << 21   # elements kept of each flat LoRA-sized buffer: 8 MB in float32
+
+
+def output_snapshot(step):
+    """What the last step returned to its caller, copied to the host: the loss, the updated LoRA
+    factors, the AdamW moments (the optimiser kernel zeroes the LoRA gradient, the first moment
+    carries it) and the optimiser state {lr, step count}.  The flat LoRA-sized buffers are sampled at
+    the same seeded positions on every run, so two builds can be compared element for element."""
+    master = step.unet.lora_master
+    n = master.numel()
+    idx = None
+    if n > DUMP_SAMPLE:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+        idx = idx.to(master.device)
+    out = {"loss": step.loss, "optimizer_state": step.opt_state}
+    for name, t in (("lora_params", master), ("adam_exp_avg", step.exp_avg), ("adam_exp_avg_sq", step.exp_avg_sq)):
+        out[name] = t if idx is None else t.index_select(0, idx)
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 # algorithmic FLOPs of one full step of ONE sample (5F + A + 4L, SURVEY 8d), by latent size
@@ -240,7 +268,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-only", action="store_true", help="one eager step, then exit (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, sampled LoRA factors and AdamW "
+                         "moments, optimiser state) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.profile_only):
+        ap.error("--dump-outputs needs the timed b200 path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -312,6 +347,8 @@ def main():
     ms_per_step = ms / args.steps
     value = world * 1e3 / ms_per_step
     loss_last = step.loss.item()
+    # taken before the passes below change the training state
+    outputs = output_snapshot(step) if args.dump_outputs and rank == 0 else None
 
     # ---- end-to-end: pinned-host inputs -> H2D -> step -> loss D2H, every step ------------
     h2d = sum(v.numel() * v.element_size() for v in host[0].values())
@@ -412,6 +449,8 @@ def main():
             "gpu_launches": int((launches_per_step or 0) * args.steps),
             "roofline": roof, "cpu_baseline": cpu,
         }
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         step.graph = step.graph_opt = None      # graphs first, then the communicator
